@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # our arm (CUDA path through the C ABI)
     python bench.py --impl reference --gpus N --steps K ...  # the reference arm: CPU path on host cores
+    python bench.py --steps K --dump-outputs DIR             # also write what the last timed step computed (DIR/*.npy)
 
 Workload (BASELINE config 2): 16 384 independent 64 KiB blocks cut from compression_66k_JSON.txt tiled to
 1 GiB, block format.  One STEP = compress all blocks, then decompress all of them (per rank).  N > 1 shards
@@ -185,6 +186,36 @@ def build_workload(nblocks: int, rank: int):
     reps = -(-(total + start) // src.size)
     data = np.tile(src, reps)[start:start + total]
     return np.ascontiguousarray(data)
+
+
+DUMP_SEED = 20260917
+DUMP_SAMPLE_BLOCKS = 64                                 # 64 x (72112 + 65536) bytes as float32: 35 MB, under 64 MB in all
+
+
+def dump_sample(nblocks: int) -> np.ndarray:
+    """Indices of the blocks whose bytes --dump-outputs writes: a fixed, seeded sample, sorted."""
+    rng = np.random.default_rng(DUMP_SEED)
+    return np.sort(rng.choice(nblocks, size=min(nblocks, DUMP_SAMPLE_BLOCKS), replace=False))
+
+
+def dump_outputs(path: str, idx, comp_rows, comp_len, comp_status, back_rows, back_len, back_status):
+    """Writes what one compress+decompress step returned to its caller as float .npy files, so that two builds can be
+    compared output for output: per-block lengths and statuses of every block, and the compressed and decompressed bytes
+    of the sampled blocks `idx` (compressed rows zeroed past each block's length: those slot bytes are not output)."""
+    os.makedirs(path, exist_ok=True)
+    comp_rows = np.asarray(comp_rows, dtype=np.float32)
+    comp_rows[np.arange(comp_rows.shape[1])[None, :] >= np.asarray(comp_len)[idx][:, None]] = 0
+    arrays = {
+        "sample_block_index": np.asarray(idx, dtype=np.float64),
+        "compressed_len": np.asarray(comp_len, dtype=np.float64),
+        "compress_status": np.asarray(comp_status, dtype=np.float64),
+        "compressed_sample": comp_rows,
+        "decompressed_len": np.asarray(back_len, dtype=np.float64),
+        "decompress_status": np.asarray(back_status, dtype=np.float64),
+        "decompressed_sample": np.asarray(back_rows, dtype=np.float32),
+    }
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 def host_topology():
@@ -414,6 +445,12 @@ def run_ours(args):
     t_end.record()
     torch.cuda.synchronize()
     k1_name, k2_name = _last_kernel(ctx, 0), _last_kernel(ctx, 1)       # what the launcher picked for the timed batches
+    if args.dump_outputs and rank == 0:
+        idx = dump_sample(nb)
+        rows = torch.from_numpy(idx).to(dev)
+        dump_outputs(args.dump_outputs, idx, d_comp.view(nb, slot)[rows].cpu().numpy(), enc.out_len.cpu().numpy(),
+                     enc.status.cpu().numpy(), d_back.view(nb, BLOCK)[rows].cpu().numpy(), dec.out_len.cpu().numpy(),
+                     dec.status.cpu().numpy())
     if world > 1:
         dist.barrier()
     clocks = sampler.stop() if rank == 0 else None
@@ -964,7 +1001,13 @@ def main():
                     help="blocks = BASELINE config 2 (default); frame = config 4 sharded frame + NCCL gather")
     ap.add_argument("--frame-blocks", type=int, default=256, help="4 MiB blocks per GPU for the sharded-frame record")
     ap.add_argument("--no-frame", action="store_true", help="skip the sharded-frame record (tuning aid)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step of the block workload computed (rank 0) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "blocks"):
+        ap.error("--dump-outputs writes the outputs of the GPU block workload (--impl ours --workload blocks)")
     if args.workload == "frame" and args.impl == "ours":
         run_frame(args)
         return

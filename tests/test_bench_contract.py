@@ -1,11 +1,13 @@
 """bench.py's contract on the CPU side: the reference arm prints one JSON line with the keys the driver reads, its
-`ms_per_step` is the timed region that `value` is computed from, and the module's helpers that need no GPU behave."""
+`ms_per_step` is the timed region that `value` is computed from, and the module's helpers that need no GPU behave.
+One GPU test checks that --dump-outputs writes what the timed step computed."""
 import json
 import os
 import subprocess
 import sys
 
 import numpy as np
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -57,3 +59,51 @@ def test_workload_is_the_tiled_fixture():
     w = bench.build_workload(8, 0)
     assert w.dtype == np.uint8 and w.size == 8 * 65536
     assert np.array_equal(w, corpus.tiled("compression_66k_JSON.txt", 8 * 65536))
+
+
+def test_dump_outputs_files(tmp_path):
+    sys.path.insert(0, ROOT)
+    import bench
+    idx = bench.dump_sample(bench.NBLOCKS_DEFAULT)
+    assert np.array_equal(idx, bench.dump_sample(bench.NBLOCKS_DEFAULT)) and np.all(np.diff(idx) > 0)
+    assert np.array_equal(bench.dump_sample(5), np.arange(5))
+    nb, slot = 8, 16
+    comp = np.arange(nb * slot, dtype=np.uint8).reshape(nb, slot)
+    clen = np.arange(nb, dtype=np.int32) + 3
+    back = np.full((nb, 4), 7, dtype=np.uint8)
+    sel = np.array([1, 6])
+    bench.dump_outputs(str(tmp_path), sel, comp[sel], clen, np.zeros(nb), back[sel], np.full(nb, 4), np.zeros(nb))
+    got = {p.stem: np.load(p) for p in tmp_path.iterdir()}
+    assert set(got) == {"sample_block_index", "compressed_len", "compress_status", "compressed_sample",
+                        "decompressed_len", "decompress_status", "decompressed_sample"}
+    assert all(a.dtype in (np.float32, np.float64) for a in got.values())
+    assert np.array_equal(got["compressed_len"], clen)
+    assert np.array_equal(got["compressed_sample"][0], np.where(np.arange(slot) < 4, comp[1], 0))
+    assert np.array_equal(got["compressed_sample"][1], np.where(np.arange(slot) < 9, comp[6], 0))
+    assert np.array_equal(got["decompressed_sample"], back[sel])
+    # at the default batch the files stay under 64 MB in all
+    k = bench.DUMP_SAMPLE_BLOCKS
+    assert 4 * k * (72112 + 65536) + 8 * (4 * bench.NBLOCKS_DEFAULT + k) < 64 << 20
+
+
+@pytest.mark.gpu
+def test_dump_outputs_are_the_timed_step(tmp_path):
+    """bench.py --dump-outputs on a small batch: the files hold what the oracle computes for the same input."""
+    sys.path.insert(0, ROOT)
+    import bench
+    import oracle
+    nb = 256
+    d = _run("--steps", "2", "--warmup", "1", "--blocks", str(nb), "--quick", "--no-frame", "--dump-outputs", str(tmp_path))
+    assert d["quick"] is True
+    got = {p.stem: np.load(p) for p in tmp_path.iterdir()}
+    data = bench.build_workload(nb, 0).reshape(nb, bench.BLOCK)
+    idx = bench.dump_sample(nb)
+    assert np.array_equal(got["sample_block_index"], idx)
+    assert not got["compress_status"].any() and not got["decompress_status"].any()
+    assert np.array_equal(got["decompressed_len"], np.full(nb, bench.BLOCK))
+    assert np.array_equal(got["decompressed_sample"], data[idx])
+    want = [oracle.compress_block(data[i].tobytes()) for i in range(nb)]
+    assert np.array_equal(got["compressed_len"], [len(w) for w in want])
+    for row, i in zip(got["compressed_sample"], idx):
+        w = np.frombuffer(want[i], dtype=np.uint8)
+        assert np.array_equal(row[:w.size], w) and not row[w.size:].any()
